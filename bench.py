@@ -3,7 +3,7 @@
 scorePairwiseConsistency() + solve() (BASELINE.json), measured the way the reference's own
 benchmark times the two calls (reference benchmarks/main.cpp:177-188).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
 
 One "step" = one full pass of the hot path over one synthetic association problem:
 score the m x m consistency graph, then run the graduated projected-gradient solver.
@@ -16,7 +16,10 @@ score the m x m consistency graph, then run the graduated projected-gradient sol
              hbm_gbs; the dense-equivalent figure (4 m^2 per pass) is reported beside it
   cpu_baseline / --impl reference : the CPU oracle (Eigen-free restatement of the reference; the
              reference cannot be built offline -- no Eigen) on this box's host cores.
-Prints exactly ONE JSON line on rank 0.
+  --dump-outputs DIR : after the timed steps, the Solution of the last timed step (u, selected nodes, F, d_final;
+             the same for the config 4 run) as DIR/<name>.npy in float64.  The inputs are seeded, so two builds run
+             with the same arguments can be compared output for output.
+Prints exactly ONE JSON line on rank 0.  Writes nothing into the source tree (it may be read-only).
 """
 import argparse
 import ctypes as C
@@ -31,6 +34,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ in the source tree
 
 METRIC = "associations/sec (scorePairwiseConsistency+solve)"
 UNIT = "associations/s"
@@ -121,6 +125,18 @@ def workload_name(name, cfg):
     return "%s: synthetic PointNormalDistance m=%d, %d%% outliers" % (name, cfg["m"], round(100 * cfg["rho"]))
 
 
+def solution_arrays(prefix, sol, u, nodes):
+    """what clp_solve_dev hands its caller, as float64 arrays (node indices are exact in float64)"""
+    return {prefix + "u": np.asarray(u, dtype=np.float64), prefix + "nodes": nodes[: sol.n_nodes].astype(np.float64),
+            prefix + "score": np.array([sol.score]), prefix + "d_final": np.array([sol.d_final])}
+
+
+def dump_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def cpu_cores():
     try:
         return len(os.sched_getaffinity(0))
@@ -191,6 +207,8 @@ def run_ours(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs is implemented for one GPU")
         from clipper_b200 import distributed as cdist
         return cdist.run_bench(args, METRIC, UNIT)
 
@@ -261,6 +279,8 @@ def run_ours(args):
     dev_ms = ev0.elapsed_time(ev1)
     value = m * args.steps / (dev_ms * 1e-3)
     nodes_dev = nodes[: sol.n_nodes].tolist(); F_dev = sol.score
+    # copied now: the host-pointer steps below write into the same `nodes` buffer
+    outputs = solution_arrays("", sol, u_out.cpu().numpy(), nodes) if args.dump_outputs else None
 
     # ---- e2e: host buffers in, Solution out, copies inside the timed region (wall clock)
     for _ in range(3):
@@ -325,7 +345,7 @@ def run_ours(args):
     # ---- BASELINE config 4 (m = 80000) on this one GPU: the N = 1 anchor of the row-sharded scaling runs
     config4 = None
     if not args.no_config4 and args.workload == "c2" and args.m is None:
-        config4 = run_config4(clipperpy, _capi, L, dev, stream, max(1, min(3, args.steps)))
+        config4 = run_config4(clipperpy, _capi, L, dev, stream, max(1, min(3, args.steps)), outputs)
 
     traffic = None
     try:
@@ -369,11 +389,14 @@ def run_ours(args):
         line["cpu_baseline"] = cpu
     if config4:
         line["config4"] = config4
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
 
 
-def run_config4(clipperpy, _capi, L, dev, stream, steps):
-    """m = 80000 (BASELINE config 4) unsharded: device-timed steps with inputs resident in HBM, same metric"""
+def run_config4(clipperpy, _capi, L, dev, stream, steps, outputs=None):
+    """m = 80000 (BASELINE config 4) unsharded: device-timed steps with inputs resident in HBM, same metric.
+    The last step's Solution goes into `outputs` (names prefixed config4_) when a dict is passed."""
     import torch
     from clipper_b200 import datagen
     prob = datagen.config_problem("c4"); cfg = prob["cfg"]; m = cfg["m"]
@@ -403,6 +426,8 @@ def run_config4(clipperpy, _capi, L, dev, stream, steps):
         step(); kms.append(sol.kernel_ms)
     ev1.record(stream); torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1)
+    if outputs is not None:
+        outputs.update(solution_arrays("config4_", sol, u_out.cpu().numpy(), nodes))
     mode = clip.dense_mode()
     kept, pass_bytes = clip.sparse_info() if mode in (3, 6) else (None, 4 * m * m)
     return {"workload": workload_name("c4", cfg), "value": m * steps / (ms * 1e-3), "unit": UNIT, "steps": steps,
@@ -426,7 +451,13 @@ def main():
     ap.add_argument("--m", type=int, default=None, help="override the workload's m (debug)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config4", action="store_true", help="skip the extra m=80000 (BASELINE config 4) measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's Solution arrays as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -4,9 +4,9 @@ The reference itself cannot be built in this image (no Eigen, DESIGN.md section 
 oracle/clipper_oracle.c -- the restatement that tests/test_oracle_golden.py pins against every fixture the reference's
 own tests hold.  They freeze that restatement: tests/test_oracle_golden.py::test_oracle_reproduces_golden_files fails if
 the oracle's arithmetic ever drifts, and tests/test_gpu_parity.py::test_cuda_path_against_golden_files compares the
-CUDA path with them on the GPU box (where /root/reference and this script's environment do not exist).
+CUDA path with them on a B200.
 
-usage:  python tests/golden/make_golden.py        (run in the build container; rewrites the .npz files)"""
+usage:  python tests/golden/make_golden.py        (rewrites the .npz files)"""
 import os
 import sys
 

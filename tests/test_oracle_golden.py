@@ -175,13 +175,17 @@ def test_dsd_rounding_in_solve():
     assert clp.dsd.solve(o.get_affinity_matrix(), supp) == s.nodes.tolist()
 
 
+# SHA-256 of the vertex payload of the reference's examples/data/bun10k.ply (the 119 904 bytes after its 235-byte
+# header: 9992 x (float32 x, y, z), little-endian), taken from the reference tree at e514dc29
+BUN10K_PLY_VERTEX_SHA256 = "0d41d0c866eb84790eb4e3943149fe8beabb8a2d3c2f441a98d180d7cf0759fb"
+
+
 def test_bunny_fixture_matches_ply():
-    # the fixture that travels to the GPU box holds exactly the vertex payload of the reference's bun10k.ply
-    import os
+    # the fixture holds exactly the vertex payload of the reference's bun10k.ply
+    import hashlib
     from clipper_b200 import datagen
     z = np.load(datagen.BUNNY_FIXTURE)["xyz"]
     assert z.shape == (9992, 3) and z.dtype == np.float32
-    if os.path.exists(datagen.REFERENCE_PLY):
-        assert np.array_equal(datagen.read_ply_xyz(datagen.REFERENCE_PLY), z)
+    assert hashlib.sha256(z.astype("<f4").tobytes()).hexdigest() == BUN10K_PLY_VERTEX_SHA256
     c = datagen.make_cloud()
     assert c.shape == (3, 9992) and abs((c.max(axis=1) - c.min(axis=1)).max() - 1.0) < 1e-12
